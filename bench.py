@@ -218,6 +218,26 @@ def sum_over_ranks(v, world, device):
     return _reduce(v, world, device, "SUM")
 
 
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, arrays, seed=0):
+    """Write what the timed path handed its caller in its last step as out_dir/<name>.npy: 8/16-bit integers as float32,
+    wider ones as float64 (both exact).  Past DUMP_LIMIT bytes in all, each array is cut to the same share of its
+    elements, picked by a generator seeded with `seed`: the same shapes give the same picks, so two builds compare
+    element for element."""
+    arrays = {k: np.asarray(v) for k, v in arrays.items()}
+    out = {k: v.astype(np.float32 if v.dtype.itemsize <= 2 else np.float64) for k, v in arrays.items()}
+    total = sum(v.nbytes for v in out.values())
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in out.items():
+        if total > DUMP_LIMIT:
+            keep = max(1, int(v.size * DUMP_LIMIT // total))
+            idx = np.sort(np.random.default_rng(seed).choice(v.size, size=keep, replace=False))
+            v = v.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, f"{k}.npy"), v)
+
+
 def timed_steps(step, steps, warmup, stream, world, local, sample_clocks=True):
     """W untimed steps, then exactly K steps bracketed by barrier + synchronize, CUDA events on the launching stream,
     max over ranks.  Returns (ms for the K steps, the running clock sampler or None): the K device-resident steps last
@@ -278,12 +298,15 @@ def run_fm(args, workload, rank, local, world, main=True):
     cap = demod.max_output(n_int16, CHUNK) + 8
     d_out = torch.empty(n_ch * cap, dtype=torch.int16, device=dev)
     stream = torch.cuda.ExternalStream(demod.stream, device=dev)
+    n_pcm = [0]
 
     def step():
-        return demod.process_device(d_in.data_ptr(), n_int16, CHUNK, d_out.data_ptr(), cap, sync=False)
+        n_pcm[0] = demod.process_device(d_in.data_ptr(), n_int16, CHUNK, d_out.data_ptr(), cap, sync=False)
 
     steps = args.steps if main else max(3, min(args.steps, 10))
     ms, sampler = timed_steps(step, steps, args.warmup, stream, world, local, sample_clocks=main)
+    if main and args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"pcm": d_out.view(n_ch, cap)[:, :n_pcm[0]].cpu().numpy()})
     stats = demod.stats()
     # dominant-kernel duration, CUDA events recorded around the fused kernel on its own stream
     kms = []
@@ -395,6 +418,9 @@ def run_power(args, workload, rank, local, world, comm, main=True):
 
     steps = args.steps if main else max(3, min(args.steps, 10))
     ms, sampler = timed_steps(step, steps, args.warmup, stream, world, local, sample_clocks=main)
+    if main and args.dump_outputs and rank == 0:
+        avg, smp = sc.read()
+        dump_outputs(args.dump_outputs, {"avg": avg, "samples": smp})
     kms = []
     for _ in range(max(3, min(steps, 10))):
         if nh > 0:
@@ -619,6 +645,7 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="only the --workload, no extra.* records")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the --workload's outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 

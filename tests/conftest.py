@@ -10,7 +10,6 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "ref: needs oracle/_ref (the compiled unmodified reference)")
 
 
 @pytest.fixture(scope="session")
@@ -19,20 +18,3 @@ def port():
     oracle.build()
     return oracle.port()
 
-
-@pytest.fixture(scope="session")
-def ref_fm():
-    import oracle
-    oracle.build()
-    if not oracle.have_ref():
-        pytest.skip("oracle/_ref not built (no /root/reference here)")
-    return oracle.RefFm()
-
-
-@pytest.fixture(scope="session")
-def ref_power():
-    import oracle
-    oracle.build()
-    if not oracle.have_ref():
-        pytest.skip("oracle/_ref not built (no /root/reference here)")
-    return oracle.RefPower()

@@ -40,26 +40,31 @@ def test_window_tables_match_port(name, port):
         assert np.array_equal(power.window_table(name, n), port.window_table(name, n))
 
 
-@pytest.mark.ref
-def test_planner_and_csv_match_reference(ref_power, port):
-    for arg, crop, boxcar, fir in [("24M:1766M:1k", 0.285, 1, 0), ("24M:1766M:1k", 0.0, 1, 0), ("88M:108M:10k", 0.1, 1, 0),
-                                   ("100M:100.2M:50", 0.0, 0, 9), ("433M:434M:100", 0.2, 1, 0), ("100M:120M:2M", 0, 1, 0)]:
-        rp = ref_power.setup(arg, crop, boxcar, fir, 0, "hamming")
+def test_planner_and_csv_match_reference(port):
+    """Plans, hop frequencies and csv_dbm() text against what the reference computed (tests/golden/ref_pin.json)."""
+    import oracle
+    pin = json.load(open(os.path.join(G, "ref_pin.json")))
+    args = [("24M:1766M:1k", 0.285, 1, 0), ("24M:1766M:1k", 0.0, 1, 0), ("88M:108M:10k", 0.1, 1, 0),
+            ("100M:100.2M:50", 0.0, 0, 9), ("433M:434M:100", 0.2, 1, 0), ("100M:120M:2M", 0, 1, 0)]
+    assert [(g["freq_arg"], g["crop_arg"], g["boxcar"], g["comp_fir_size"]) for g in pin["planner"]] == args
+    for (arg, crop, boxcar, fir), rp in zip(args, pin["planner"]):
         plan = power.plan_range(arg, crop, boxcar, fir, 0)
         assert (plan.n_hops, plan.bin_e, plan.buf_len, plan.downsample, plan.downsample_passes, plan.rate) == \
-            (rp.tune_count, rp.bin_e, rp.buf_len, rp.downsample, rp.downsample_passes, rp.rate), arg
-        assert abs(plan.crop - rp.crop) < 1e-15
-        freqs = ref_power.hop_freqs()
-        assert [plan.hop_freq(i) for i in range(plan.n_hops)] == [int(f) for f in freqs]
+            (rp["tune_count"], rp["bin_e"], rp["buf_len"], rp["downsample"], rp["downsample_passes"], rp["rate"]), arg
+        assert abs(plan.crop - rp["crop"]) < 1e-15
+        freqs = np.array([plan.hop_freq(i) for i in range(plan.n_hops)], dtype=np.int64)
+        assert digest(freqs) == rp["hop_freqs_sha256"]
     # CSV text identical for the same accumulators
-    rp = ref_power.setup("24M:60M:1k", 0.285, 1, 0, 0, "hamming")
-    rng = np.random.default_rng(5)
-    x = rng.integers(-100, 101, size=(2, rp.tune_count, rp.buf_len), dtype=np.int32).astype(np.int16)
-    avg, smp = ref_power.scan(x, 2)
-    plan = power.plan_range("24M:60M:1k", 0.285)
+    g = pin["csv"]
+    plan = power.plan_range(g["freq_arg"], g["crop"])
+    rng = np.random.default_rng(g["seed"])
+    x = rng.integers(-100, 101, size=(2, plan.n_hops, plan.buf_len), dtype=np.int32).astype(np.int16)
+    pp = oracle.PowerParams(bin_e=plan.bin_e, buf_len=plan.buf_len, downsample=plan.downsample,
+                            downsample_passes=plan.downsample_passes)
+    avg, smp = port.power_scan(pp, port.window_table("hamming", 1 << plan.bin_e), x, 2, plan.n_hops)
+    assert digest(avg) == g["avg_sha256"] and [int(v) for v in smp] == g["samples"]
     mine = power.csv_rows(plan, avg, smp)
-    theirs = ref_power.csv("/tmp/_csv_ref.txt")
-    assert mine == theirs
+    assert digest(np.frombuffer(mine.encode(), dtype=np.uint8)) == g["text_sha256"]
 
 
 def test_wbfm_preset_keeps_a_later_squelch_level():
